@@ -1,17 +1,16 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the batched CrowdSim-v0 step path on B200 (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--envs 4096] [--humans 5]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--envs 4096] [--humans 5] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[1] = 4096 batched envs x 5 ORCA humans, circle_crossing, ORCA robot,
-robot invisible, per GPU. One bench "step" = one lockstep pass of the hot path over one 4096-env batch: the fused step
-kernel (6 ORCA solves/env, collision/reward/terminal, integration, episode bookkeeping) plus on-device re-generation
-of the scenes of envs whose episode just ended (fresh MT19937 seeds), so every env is live on every step.
-Because 4096 envs of state are only 2.6 MB, the bench rotates through POOLS independent batches whose combined state
-exceeds the 126 MB L2 ("inputs larger than L2"); the batch touched by a step was last touched POOLS steps ago.
-The timed region is ONE CUDA graph of K step launches (+ one scene-prefetch launch per batch on every 4th visit, side
-streams); batch p always runs on stream p mod S (--streams, default 16), so the steps of one batch stay ordered while
-independent batches overlap on the device. `value` = env-steps PERFORMED (counted by the step kernel) / device time;
+robot invisible, per GPU. Because 4096 envs of state are only 2.6 MB, the bench holds POOLS independent batches whose
+combined state exceeds the 126 MB L2 ("inputs larger than L2"). One bench "step" = one call of the hot path on every
+batch: crowdsim_step_n advances each env by C env-steps (--chunk, default 16) in one launch of the fused step kernel (6
+ORCA solves/env, collision/reward/terminal, integration, episode bookkeeping), and one scene-prefetch launch per batch on
+a side stream re-generates the scenes of envs whose episode ended (fresh MT19937 seeds), so every env is live on every
+env-step. The timed region is exactly K such steps; batch p always runs on stream p mod S (--streams, default 16), so the
+steps of one batch stay ordered while independent batches overlap on the device. `value` = env-steps PERFORMED (counted by the step kernel) / device time;
 `single_stream` = the same with one batch in flight; `e2e` = HostStepper.launch()/wait() over 16 batches with pinned host
 buffers in and out on every batch-step; `roofline` = the step kernel alone (single-stream graph, CUDA events).
 
@@ -40,8 +39,8 @@ ALG_BYTES = lambda n: 8 * (19 + 12 * n) + 2      # SURVEY.md 8(d): 634 B at N=5,
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=25600)
-    ap.add_argument('--warmup', type=int, default=2560)
+    ap.add_argument('--steps', type=int, default=25, help='timed steps; one step advances every env on the GPU by --chunk env-steps')
+    ap.add_argument('--warmup', type=int, default=24, help='steps before the timed region (at least 384 env-steps per env: a steady mix of episode phases)')
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--envs', type=int, default=4096, help='envs per batch per GPU')
     ap.add_argument('--humans', type=int, default=5)
@@ -55,7 +54,12 @@ def parse():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-python-loop', action='store_true', help='reference arm: skip the reference-shaped Python loop timing')
     ap.add_argument('--no-scale', action='store_true', help='skip the supplementary 1 Mi-env launch measurement')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps, write a seeded sample of the per-case episode '
+                    'rows the timed path recorded as DIR/<name>.npy (float64), for comparing two builds output for output')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be >= 1')
+    return args
 
 
 def load_peaks():
@@ -259,9 +263,34 @@ def cpu_oracle_rate(args, seconds=10.0):
 
 
 # ----------------------------------------------------------------------------------------------------------------------
-def _lcm(a, b):
-    import math
-    return a * b // math.gcd(a, b)
+DUMP_ROWS = 16384
+
+
+def dump_episode_rows(out_dir, envs, B):
+    """--dump-outputs: the per-case episode rows the step kernel of the timed path recorded (what Explorer.run_k_episodes
+    hands its caller: terminal info, steps, time, discounted return, danger count, min-distance sum, final robot position),
+    for a fixed seeded sample of DUMP_ROWS of the first 2 x B cases of every batch (claimed by the initial reset and the
+    first scene prefetch). A row depends only on its case's seed, not on which env slot ran the case or when, so with the
+    same arguments the files are identical from run to run; the slot-level state after the last step is not, because the
+    scene refills race the steps by design. Those cases have all ended: an episode lasts at most ~100 steps and the
+    warm-up alone is 384."""
+    import numpy as np
+    import torch
+    rng = np.random.RandomState(0)
+    per = max(1, DUMP_ROWS // len(envs))
+    cols = {k: [] for k in ('seed', 'info', 'steps', 'time', 'return', 'too_close', 'min_dist_sum', 'final_robot_pos')}
+    for env in envs:
+        idx = torch.from_numpy(np.sort(rng.choice(2 * B, min(per, 2 * B), replace=False))).to(env.device)
+        ep = env.episodes
+        if not bool((ep.res_steps[idx] > 0).all()):
+            raise RuntimeError('--dump-outputs: a sampled case has not ended')
+        cols['seed'].append((idx + env._seed_base).double())          # MT19937 seed of the case (train phase: 2000 + case)
+        for k, a in (('info', ep.res_info), ('steps', ep.res_steps), ('time', ep.res_time), ('return', ep.res_return),
+                     ('too_close', ep.res_too_close), ('min_dist_sum', ep.res_min_dist_sum), ('final_robot_pos', ep.res_final_rpos)):
+            cols[k].append(a[idx].double())
+    os.makedirs(out_dir, exist_ok=True)
+    for k, parts in cols.items():
+        np.save(os.path.join(out_dir, 'episode_%s.npy' % k), torch.cat(parts).cpu().numpy())
 
 
 def run_ours(args):
@@ -284,21 +313,16 @@ def run_ours(args):
     pools = args.pools or max(2, int(1.3 * 126e6 / (B * bytes_per_env)) + 1)
     S = max(1, min(args.streams, pools))
     pools = (pools + S - 1) // S * S                         # every stream owns the same number of batches
-    round_steps = pools * C                                  # bench steps of one round (every batch advanced by C steps)
 
     def barrier():
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
 
-    # ---- how many steps get timed: R back-to-back replays of K steps, no gap between them (the streams are only joined
-    # at the two ends of the region), R >= 200 for short K and long enough for >= ~80 ms; whole rounds only ----
-    est_us_per_step = 2.0
-    unit = _lcm(K, round_steps)
-    want_steps = max(200 * K if K <= 4096 else K, int(0.08 / (est_us_per_step * 1e-6)))
-    timed_steps = min((want_steps + unit - 1) // unit * unit, max(unit, 4_000_000 // unit * unit))
-    rounds = timed_steps // round_steps
-    warm_rounds = max(24, (max(W, 3) + round_steps - 1) // round_steps)     # >= 24 x C = 192 steps per batch: steady episode mix
+    # ---- the timed region: exactly K rounds (every batch advanced by C env-steps in one launch), no gap between them; the
+    # streams are only joined at the two ends of the region ----
+    rounds = K
+    warm_rounds = max(W, -(-384 // C))                       # >= 384 env-steps per env: steady episode mix
 
     envs = []
     for p in range(pools):
@@ -377,17 +401,9 @@ def run_ours(args):
             tot += int(env.episodes.res_steps[:n].sum().item()) + int((env.episodes.ep_steps * env.state.active.to(torch.int32)).sum().item())
         return tot
 
-    # ---- warm-up: every batch far into steady state (>= 192 steps, i.e. several episode lengths: the mix of episode phases is
-    # stationary), then a few timed rounds to size the region ----
+    # ---- warm-up: every batch far into steady state (>= 384 env-steps, i.e. several episode lengths: the mix of episode
+    # phases is stationary) ----
     run_rounds(warm_rounds)
-    torch.cuda.synchronize()
-    a0, a1 = run_rounds(4)
-    torch.cuda.synchronize()
-    est_us_per_step = 1e3 * a0.elapsed_time(a1) / (4 * round_steps)
-    want_steps = max(200 * K if K <= 4096 else K, int(0.08 / (est_us_per_step * 1e-6)))
-    timed_steps = min((want_steps + unit - 1) // unit * unit, rounds * round_steps)
-    rounds = timed_steps // round_steps
-    warm_done = (warm_rounds + 4) * round_steps
 
     barrier()
     steps_before = env_steps_done()
@@ -397,6 +413,8 @@ def run_ours(args):
     e0, e1 = run_rounds(rounds, tick=ticks)
     barrier()
     sampler.mark_stop()
+    if args.dump_outputs and rank == 0:
+        dump_episode_rows(args.dump_outputs, envs, B)
     launches = rounds * launches_per_round
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop()
@@ -408,14 +426,14 @@ def run_ours(args):
         dist.all_reduce(cnt, op=dist.ReduceOp.SUM)
     ms_max = float(t.item())
     live_total = int(cnt.item())
-    value = live_total / (ms_max * 1e-3)                     # == world * B * timed_steps / time unless envs were parked
+    value = live_total / (ms_max * 1e-3)                     # == world * pools * B * C * K / time unless envs were parked
     # distribution over the rounds (stream 0's clock): a steady region has median ~ mean
     rt = sorted(ticks[i].elapsed_time(ticks[i + 1]) for i in range(len(ticks) - 1)) if len(ticks) > 2 else []
     round_stats = None
     if rt:
         med = rt[len(rt) // 2]
-        round_stats = {'rounds': rounds, 'steps_per_round': round_steps, 'median_ms': med, 'p10_ms': rt[len(rt) // 10], 'p90_ms': rt[(9 * len(rt)) // 10],
-                       'median_value': world * B * round_steps / (med * 1e-3),
+        round_stats = {'rounds': rounds, 'env_steps_per_env': C, 'median_ms': med, 'p10_ms': rt[len(rt) // 10], 'p90_ms': rt[(9 * len(rt)) // 10],
+                       'median_value': world * pools * B * C / (med * 1e-3),
                        'note': 'per-round durations on stream 0 of rank 0 (every batch advanced by %d steps per round); median_value = nominal env-steps of a round / median' % C}
 
     # ---- the path's single collective: gather of episode statistics (terminal-class counts + env-steps of all finished
@@ -638,19 +656,19 @@ def run_ours(args):
 
     if rank == 0:
         line = {'metric': METRIC, 'value': value, 'unit': 'env-steps/s', 'n_gpus': world, 'steps': K, 'warmup': W,
-                'ms_per_step': ms_max / timed_steps, 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None,
+                'ms_per_step': ms_max / K, 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None,
                 'dtype': 'f64 state + f32 ORCA solver', 'data': 'synthetic',
                 'config': {'workload': WORKLOAD % (B, N, args.rule),
                            'envs_per_gpu': B, 'humans': N, 'l2': 'inputs larger than L2: %d rotating independent batches = %.0f MB of state' % (pools, pools * B * bytes_per_env / 1e6),
                            'batches_in_flight': S, 'steps_per_launch': C,
                            'parallelism': 'independent envs sharded over %d GPU(s), no data-path collective' % world},
                 'value_is': '%d independent %d-env batches in flight on %d streams (weak scaling unit = one GPU with its %d batches); the config-literal one-batch number is `single_batch`' % (S, B, S, pools),
-                'timed_region': {'replays': timed_steps // K, 'steps_per_replay': K, 'timed_steps': timed_steps, 'ms': ms_max,
-                                 'warmup_steps_done': warm_done,
-                                 'note': 'replays of K steps run back to back without a gap (streams joined only at the two ends of the region); ms_per_step = ms / timed_steps; '
-                                         'every batch was advanced >= %d steps before the region (steady mix of episode phases)' % (warm_done // pools)},
+                'timed_region': {'timed_steps': K, 'envs_per_step': pools * B, 'env_steps_per_env_per_step': C, 'ms': ms_max,
+                                 'warmup_steps_done': warm_rounds,
+                                 'note': 'K steps (one crowdsim_step_n launch per batch each) run back to back without a gap (streams joined only at the two ends of the region); ms_per_step = ms / K; '
+                                         'every env was advanced %d env-steps before the region (steady mix of episode phases)' % (warm_rounds * C)},
                 'rounds': round_stats,
-                'env_steps': {'performed': live_total, 'nominal': world * B * timed_steps,
+                'env_steps': {'performed': live_total, 'nominal': world * pools * B * C * K,
                               'note': 'value = performed / time; performed is counted by the step kernel (episode step counters), nominal = envs x steps; they differ only if envs waited for a scene refill'},
                 'clocks': clocks, 'gpu_launches': int(launches), 'gpu_launches_note': launches_note,
                 'e2e': {'value': e2e_value, 'unit': 'env-steps/s', 'h2d_bytes_per_step': h2d, 'd2h_bytes_per_step': d2h,

@@ -15,6 +15,7 @@ What is recorded (floats as repr() strings, exact round trip):
   rotate.json    CADRL.rotate + one-step lookahead inputs/outputs of MultiHumanRL.predict's inner loop
   occupancy_maps.json  MultiHumanRL.build_occupancy_maps on scene / lookahead / random human states
   policy_decisions.json  per-action values and greedy actions of the reference's CADRL / LSTM-RL policies
+  network_ports.json     outputs of the reference's value-network modules with seeded weights loaded
 
 usage: python oracle/gen_golden.py [--quick]
 """
@@ -48,6 +49,10 @@ from crowd_sim.envs.utils.state import JointState  # noqa: E402
 from crowd_sim.envs.policy.orca import ORCA  # noqa: E402
 from crowd_nav.utils.explorer import Explorer  # noqa: E402
 from crowd_nav.policy.policy_factory import policy_factory  # noqa: E402
+from crowd_nav.policy import cadrl, lstm_rl, sarl  # noqa: E402
+
+sys.path.insert(0, os.path.join(ROOT, 'tests'))
+from util import network_port_input, network_port_weights  # noqa: E402
 
 OUT = os.path.join(ROOT, 'tests', 'golden')
 INFO_CODE = {Nothing: 0, Danger: 1, ReachGoal: 2, Collision: 3, Timeout: 4}
@@ -431,7 +436,36 @@ def run_human_times():
         json.dump({'rows': rows}, f, separators=(',', ':'))
 
 
+NETWORK_PORTS = (  # name, the reference's module with the policy.config defaults (crowd_nav/policy/*.py)
+    ('lstm_rl_v1', lambda: lstm_rl.ValueNetwork1(13, 6, [150, 100, 100, 1], 50)),
+    ('lstm_rl_v2', lambda: lstm_rl.ValueNetwork2(13, 6, [150, 100, 100, 50], [150, 100, 100, 1], 50)),
+    ('sarl', lambda: sarl.ValueNetwork(13, 6, [150, 100], [100, 50], [150, 100, 100, 1], [100, 100, 1], True, 1.0, 4)),
+    ('cadrl', lambda: cadrl.ValueNetwork(13, [150, 100, 100, 1])),
+)
+
+
+def run_network_ports():
+    """Outputs of the reference's value-network modules (LSTM-RL without / with interaction module, SARL, CADRL) with
+    seeded stand-in weights loaded (network_port_weights), on a seeded input; CADRL sees the first human's rows only."""
+    x = network_port_input()
+    out = {}
+    for i, (name, make) in enumerate(NETWORK_PORTS):
+        net = make()
+        keys_shapes = [(k, list(v.shape)) for k, v in net.state_dict().items()]
+        net.load_state_dict(network_port_weights(keys_shapes, 100 + i))
+        with torch.no_grad():
+            y = net(x[:, 0] if name == 'cadrl' else x)
+        out[name] = {'seed': 100 + i, 'keys_shapes': keys_shapes, 'output': [[R(v) for v in row] for row in y.tolist()]}
+    with gzip.open(os.path.join(OUT, 'network_ports.json.gz'), 'wt') as f:
+        json.dump(out, f, separators=(',', ':'))
+    print('network ports', {k: len(v['keys_shapes']) for k, v in out.items()})
+
+
 def main():
+    if '--network-ports-only' in sys.argv:
+        os.makedirs(OUT, exist_ok=True)
+        run_network_ports()
+        return
     if '--human-times-only' in sys.argv:
         os.makedirs(OUT, exist_ok=True)
         run_human_times()
@@ -477,6 +511,7 @@ def main():
     run_policy_decisions()
     run_rl_memory()
     run_human_times()
+    run_network_ports()
 
 
 if __name__ == '__main__':

@@ -47,6 +47,20 @@ def fill_host_state(po, scenes, N):
     return st
 
 
+def network_port_weights(keys_shapes, seed):
+    """Seeded weights for a state_dict layout [(key, shape)]: float32 uniform(-0.2, 0.2), one numpy RandomState draw per
+    key in the given order (golden network_ports: loaded into the reference's modules and into the ports alike)."""
+    import torch
+    rng = np.random.RandomState(seed)
+    return {k: torch.from_numpy(rng.uniform(-0.2, 0.2, shape).astype(np.float32)) for k, shape in keys_shapes}
+
+
+def network_port_input():
+    """[9 states][5 humans][13] float32 rows for the value networks (golden network_ports)."""
+    import torch
+    return torch.from_numpy(np.random.RandomState(12345).standard_normal((9, 5, 13)).astype(np.float32))
+
+
 def ulp_diff(a, b):
     """Elementwise distance in float64 ulps (for values of equal sign / finite)."""
     a = np.ascontiguousarray(a, dtype=np.float64); b = np.ascontiguousarray(b, dtype=np.float64)
