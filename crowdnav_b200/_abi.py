@@ -7,12 +7,14 @@ for its CPU library. No torch types cross the boundary.
 import ctypes as C
 import os
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 MAX_HUMANS = 63
 MAX_NEIGHBORS = 10
 
 INFO_NOTHING, INFO_DANGER, INFO_REACHGOAL, INFO_COLLISION, INFO_TIMEOUT = 0, 1, 2, 3, 4
-ROBOT_EXTERNAL_XY, ROBOT_ORCA, ROBOT_EXTERNAL_ROT = 0, 1, 2
+ROBOT_EXTERNAL_XY, ROBOT_ORCA, ROBOT_EXTERNAL_ROT, ROBOT_LINEAR = 0, 1, 2, 3
+HUMANS_ORCA, HUMANS_LINEAR = 0, 1   # crowdsim_params.human_policy (env.config [humans] policy)
+HUMAN_POLICIES = {'orca': HUMANS_ORCA, 'linear': HUMANS_LINEAR}
 RULE_CIRCLE, RULE_SQUARE = 0, 1
 RULE_MIXED = 2
 PARKED_X = 1.0e6                  # include/crowdsim_b200.h: CROWDSIM_PARKED_X
@@ -28,7 +30,8 @@ class Params(C.Structure):
                 ('discomfort_penalty_factor', C.c_double), ('neighbor_dist', C.c_double),
                 ('time_horizon', C.c_double), ('max_neighbors', C.c_int32),
                 ('human_safety_space', C.c_double), ('robot_safety_space', C.c_double),
-                ('robot_visible', C.c_int32), ('robot_policy', C.c_int32)]
+                ('robot_visible', C.c_int32), ('robot_policy', C.c_int32),
+                ('human_policy', C.c_int32)]       # last: the 13-argument positional form keeps meaning ORCA humans
 
 
 class State(C.Structure):
@@ -147,5 +150,5 @@ def check(rc, what):
     if rc != 0:
         if rc > 0:
             raise RuntimeError('%s: CUDA error %d' % (what, rc))
-        raise ValueError('%s: %s' % (what, {-1: 'invalid argument', -2: 'unsupported size',
+        raise ValueError('%s: %s' % (what, {-1: 'invalid argument', -2: 'unsupported size or policy',
                                              -3: 'no sm_100 CUDA device'}.get(rc, 'error %d' % rc)))

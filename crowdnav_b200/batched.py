@@ -171,6 +171,7 @@ class BatchedCrowdSim(object):
         self.robot_visible = False; self.robot_radius = 0.3; self.robot_v_pref = 1.0
         self.human_radius = 0.3; self.human_v_pref = 1.0
         self.robot_policy = _abi.ROBOT_ORCA
+        self.human_policy = _abi.HUMANS_ORCA
         self.human_safety_space = 0.0; self.robot_safety_space = 0.0
         # ORCA constants (orca.py:61-64)
         self.neighbor_dist = 10.0; self.max_neighbors = 10; self.time_horizon = 5.0
@@ -189,8 +190,11 @@ class BatchedCrowdSim(object):
         self.collision_penalty = config.getfloat('reward', 'collision_penalty')
         self.discomfort_dist = config.getfloat('reward', 'discomfort_dist')
         self.discomfort_penalty_factor = config.getfloat('reward', 'discomfort_penalty_factor')
-        if config.get('humans', 'policy') != 'orca':
+        # env.config [humans] policy (policy_factory.py:9-12): 'orca' or 'linear' (straight to the goal, ignores everyone)
+        human_policy = config.get('humans', 'policy')
+        if human_policy not in _abi.HUMAN_POLICIES:
             raise NotImplementedError
+        self.human_policy = _abi.HUMAN_POLICIES[human_policy]
         u32max = int(np.iinfo(np.uint32).max)
         self.case_capacity = {'train': u32max - 2000, 'val': 1000, 'test': 1000}
         self.case_size = {'train': u32max - 2000, 'val': config.getint('env', 'val_size'),
@@ -222,14 +226,20 @@ class BatchedCrowdSim(object):
         self._seed32 = torch.zeros(B, dtype=torch.int32, device=self.device)
 
     def set_robot_policy(self, kind):
-        self.robot_policy = {'orca': _abi.ROBOT_ORCA, 'external_xy': _abi.ROBOT_EXTERNAL_XY, 'holonomic': _abi.ROBOT_EXTERNAL_XY,
-                             'external_rot': _abi.ROBOT_EXTERNAL_ROT, 'unicycle': _abi.ROBOT_EXTERNAL_ROT}[kind]
+        """'orca' / 'linear': the robot decides inside the step kernel (ORCA.predict / Linear.predict of its pre-step state);
+        'external_xy' ('holonomic') / 'external_rot' ('unicycle'): step() takes the robot's actions."""
+        self.robot_policy = {'orca': _abi.ROBOT_ORCA, 'linear': _abi.ROBOT_LINEAR, 'external_xy': _abi.ROBOT_EXTERNAL_XY,
+                             'holonomic': _abi.ROBOT_EXTERNAL_XY, 'external_rot': _abi.ROBOT_EXTERNAL_ROT,
+                             'unicycle': _abi.ROBOT_EXTERNAL_ROT}[kind]
+
+    def robot_decides_on_device(self):
+        return self.robot_policy in (_abi.ROBOT_ORCA, _abi.ROBOT_LINEAR)
 
     def params(self):
         return _abi.Params(self.time_step, float(self.time_limit), self.success_reward, self.collision_penalty,
                            self.discomfort_dist, self.discomfort_penalty_factor, self.neighbor_dist, self.time_horizon,
                            self.max_neighbors, self.human_safety_space, self.robot_safety_space,
-                           int(bool(self.robot_visible)), self.robot_policy)
+                           int(bool(self.robot_visible)), self.robot_policy, self.human_policy)
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
@@ -315,11 +325,11 @@ class BatchedCrowdSim(object):
 
     # ---- step ----------------------------------------------------------------------------------------------------
     def step(self, actions=None, n_steps=1):
-        """One lockstep env-step. `actions` [B][2] float64 device tensor (vx,vy) / (v,r); None when the robot runs ORCA.
-        n_steps > 1: crowdsim_step_n -- exactly n_steps single steps; with an ORCA robot and N <= 5 they run inside ONE
+        """One lockstep env-step. `actions` [B][2] float64 device tensor (vx,vy) / (v,r); None when the robot runs ORCA or
+        Linear. n_steps > 1: crowdsim_step_n -- exactly n_steps single steps; with an ORCA / Linear robot and N <= 5 they run inside ONE
         kernel launch with the state in registers (the closed episode loop of explorer.py:41-43). The returned reward /
         done / info are those of each env's last live step."""
-        if self.robot_policy != _abi.ROBOT_ORCA:
+        if not self.robot_decides_on_device():
             if actions is None:
                 raise ValueError('robot policy is external: actions required')
             if actions.data_ptr() != self.action.data_ptr():
@@ -344,7 +354,7 @@ class BatchedCrowdSim(object):
         return self.observation(), self.reward, self.done, self.info
 
     def step_n(self, n_steps):
-        """n_steps closed-loop env-steps (ORCA robot): see step()."""
+        """n_steps closed-loop env-steps (ORCA or Linear robot): see step()."""
         return self.step(None, n_steps=n_steps)
 
     def orca_act(self, out=None):
@@ -602,7 +612,7 @@ class HostStepperGroup(object):
 
 
 def default_config(human_num=5, test_sim='circle_crossing', train_val_sim='circle_crossing', robot_visible=False,
-                   randomize_attributes=False):
+                   randomize_attributes=False, human_policy='orca'):
     """The reference's crowd_nav/configs/env.config:1-37 as a RawConfigParser (values restated, not read from disk)."""
     import configparser
     cfg = configparser.RawConfigParser()
@@ -613,7 +623,7 @@ def default_config(human_num=5, test_sim='circle_crossing', train_val_sim='circl
                    'discomfort_penalty_factor': '0.5'},
         'sim': {'train_val_sim': train_val_sim, 'test_sim': test_sim, 'square_width': '10', 'circle_radius': '4',
                 'human_num': str(human_num)},
-        'humans': {'visible': 'true', 'policy': 'orca', 'radius': '0.3', 'v_pref': '1', 'sensor': 'coordinates'},
+        'humans': {'visible': 'true', 'policy': human_policy, 'radius': '0.3', 'v_pref': '1', 'sensor': 'coordinates'},
         'robot': {'visible': 'true' if robot_visible else 'false', 'policy': 'none', 'radius': '0.3', 'v_pref': '1',
                   'sensor': 'coordinates'},
     })

@@ -27,6 +27,36 @@ __device__ __forceinline__ double point_to_segment_dist0(double x1, double y1, d
     return norm2(x, y);
 }
 
+// Linear.predict (crowd_sim/envs/policy/linear.py:15-22): straight to the goal at v_pref, float64 like numpy. An agent standing
+// on its goal gets atan2(0, 0) = 0, i.e. it steps +x, as the reference's does.
+__device__ __forceinline__ double2 linear_velocity(double2 pos, double2 goal, double v_pref)
+{
+    const double th = atan2(goal.y - pos.y, goal.x - pos.x);
+    return make_double2(cos(th) * v_pref, sin(th) * v_pref);
+}
+// The same for a human slot; the PARKED slots of rule `mixed` (include/crowdsim_b200.h) never move.
+__device__ __forceinline__ double2 linear_human_velocity(double2 pos, double2 goal, double v_pref)
+{
+    if (pos.x >= CROWDSIM_PARKED_X / 2) return make_double2(0, 0);
+    return linear_velocity(pos, goal, v_pref);
+}
+
+// Policy selection of the step / lookahead kernels: a compile-time bit set (template parameter LIN), so that the ORCA-human
+// instantiations carry no code of the linear ones.
+constexpr int kLinHumans = 1;   // human_policy == CROWDSIM_HUMANS_LINEAR
+constexpr int kLinRobot = 2;    // robot_policy == CROWDSIM_ROBOT_LINEAR
+
+// Host-side validation of the policy fields of crowdsim_params.
+inline bool policies_supported(const crowdsim_params *p)
+{
+    return p->robot_policy >= CROWDSIM_ROBOT_EXTERNAL_XY && p->robot_policy <= CROWDSIM_ROBOT_LINEAR &&
+           (p->human_policy == CROWDSIM_HUMANS_ORCA || p->human_policy == CROWDSIM_HUMANS_LINEAR);
+}
+inline int lin_bits(const crowdsim_params *p)
+{
+    return (p->human_policy == CROWDSIM_HUMANS_LINEAR ? kLinHumans : 0) | (p->robot_policy == CROWDSIM_ROBOT_LINEAR ? kLinRobot : 0);
+}
+
 __device__ __forceinline__ double2 ld2(const double *p, size_t i) { return reinterpret_cast<const double2 *>(p)[i]; }
 __device__ __forceinline__ void st2(double *p, size_t i, double2 v) { reinterpret_cast<double2 *>(p)[i] = v; }
 __device__ __forceinline__ double2 ld2_cg(const double *p, size_t i) { return __ldcg(reinterpret_cast<const double2 *>(p) + i); }

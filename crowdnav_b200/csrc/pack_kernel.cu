@@ -13,6 +13,7 @@
 // functions (the reference's are torch CPU's), so parity on these rows is a 1e-5 tolerance, not bit-exact.
 // Output of one env is A*N*13 contiguous floats: it is assembled in a shared-memory tile and written back with
 // fully coalesced stores.
+#include <type_traits>
 #include "crowdsim_common.cuh"
 
 namespace cs {
@@ -72,8 +73,11 @@ struct LookArgs {
     double *out_reward;
 };
 
+// HLIN: the humans follow Linear.predict (float64 velocities, kept as such for the next positions) instead of ORCA.
+template <bool HLIN = false>
 __global__ void __launch_bounds__(256) lookahead_kernel(const __grid_constant__ LookArgs G)
 {
+    using HVel = typename std::conditional<HLIN, double2, float2>::type;
     extern __shared__ __align__(16) unsigned char smem[];
     const int T = blockDim.x, tid = threadIdx.x;
     const int N = G.N, L = G.L, A = G.A;
@@ -85,7 +89,7 @@ __global__ void __launch_bounds__(256) lookahead_kernel(const __grid_constant__ 
     double2 *s_rattr = reinterpret_cast<double2 *>(xp); xp += (size_t)G.EPB * 16;    // robot radius, v_pref
     double2 *s_thtime = reinterpret_cast<double2 *>(xp); xp += (size_t)G.EPB * 16;   // robot theta, global_time
     double2 *s_actions = reinterpret_cast<double2 *>(xp); xp += (size_t)A * 16;
-    float2 *s_nvel = reinterpret_cast<float2 *>(xp); xp += (size_t)G.EPB * L * 8;     // human ORCA actions
+    HVel *s_nvel = reinterpret_cast<HVel *>(xp); xp += (size_t)G.EPB * L * sizeof(HVel);  // human actions
     float *tile = reinterpret_cast<float *>(xp);                                      // [A][N][13]
 
     const int le = tid / L, a = tid - le * L;
@@ -107,8 +111,8 @@ __global__ void __launch_bounds__(256) lookahead_kernel(const __grid_constant__ 
     __syncthreads();
 
     if (live && !is_robot) {
-        const orca::V2 nv = orca_predict(s, k, le, a, N, L, pos, goal, attr.y, tid, T);
-        s_nvel[tid] = make_float2(nv.x, nv.y);
+        if constexpr (HLIN) s_nvel[tid] = linear_human_velocity(pos, goal, attr.y);
+        else { const orca::V2 nv = orca_predict(s, k, le, a, N, L, pos, goal, attr.y, tid, T); s_nvel[tid] = make_float2(nv.x, nv.y); }
     }
     __syncthreads();
 
@@ -155,11 +159,11 @@ __global__ void __launch_bounds__(256) lookahead_kernel(const __grid_constant__ 
             rotate_self(fpx, fpy, (float)nvx, (float)nvy, (float)rg.x, (float)rg.y, c, sn, rot, dg, rvx, rvy);
             const float th_out = G.unicycle ? ((float)nth - rot) : 0.f;
             for (int i = 0; i < N; ++i) {
-                const double2 hp = s.pos64[base + i]; const float2 hn = s_nvel[base + i];
+                const double2 hp = s.pos64[base + i]; const HVel hn = s_nvel[base + i];
                 // agent.py:63-74 get_next_observable_state(human_action)
                 const double nhx = hp.x + (double)hn.x * dt, nhy = hp.y + (double)hn.y * dt;
                 rotate_row(tile + (size_t)kk * row_floats + i * 13, fpx, fpy, (float)ra.x, (float)ra.y, th_out, dg, rvx, rvy, c, sn,
-                           (float)nhx, (float)nhy, hn.x, hn.y, (float)s.rad64[base + i]);
+                           (float)nhx, (float)nhy, (float)hn.x, (float)hn.y, (float)s.rad64[base + i]);
             }
         }
         __syncthreads();
@@ -175,6 +179,7 @@ __global__ void __launch_bounds__(256) lookahead_kernel(const __grid_constant__ 
 // CURRENT state, nothing mutated. Same staging and solver as the lookahead kernel. ----
 struct NextArgs { KParams k; int B, N, L, EPB; crowdsim_state st; double *next_pos, *next_vel; };
 
+template <bool HLIN = false>
 __global__ void __launch_bounds__(256) lookahead_humans_kernel(const __grid_constant__ NextArgs G)
 {
     extern __shared__ __align__(16) unsigned char smem[];
@@ -194,8 +199,9 @@ __global__ void __launch_bounds__(256) lookahead_humans_kernel(const __grid_cons
     stage_agent(s, k, tid, pos, vel, attr.x);
     __syncthreads();
     if (live && !is_robot) {
-        const orca::V2 nv = orca_predict(s, k, le, a, N, L, pos, goal, attr.y, tid, T);
-        const double hx = (double)nv.x, hy = (double)nv.y;
+        double hx, hy;
+        if constexpr (HLIN) { const double2 lv = linear_human_velocity(pos, goal, attr.y); hx = lv.x; hy = lv.y; }
+        else { const orca::V2 nv = orca_predict(s, k, le, a, N, L, pos, goal, attr.y, tid, T); hx = (double)nv.x; hy = (double)nv.y; }
         const size_t i = (size_t)e * N + a;
         st2(G.next_pos, i, make_double2(pos.x + hx * k.time_step, pos.y + hy * k.time_step));
         st2(G.next_vel, i, make_double2(hx, hy));
@@ -263,7 +269,7 @@ extern "C" int crowdsim_lookahead_pack(const crowdsim_params *prm, int B, int N,
                                        float *out_states, double *out_reward, void *stream)
 {
     if (!prm || !st || !actions || !out_states || !out_reward || B < 0 || N < 1 || A < 1) return CROWDSIM_EINVAL;
-    if (N > CROWDSIM_MAX_HUMANS || prm->max_neighbors > CROWDSIM_MAX_NEIGHBORS) return CROWDSIM_EUNSUPPORTED;
+    if (N > CROWDSIM_MAX_HUMANS || prm->max_neighbors > CROWDSIM_MAX_NEIGHBORS || !cs::policies_supported(prm)) return CROWDSIM_EUNSUPPORTED;
     if (!st->h_pos || !st->h_vel || !st->h_goal || !st->h_attr || !st->r_pos || !st->r_vel || !st->r_goal || !st->r_attr || !st->g_time) return CROWDSIM_EINVAL;
     if (kinematics_unicycle && !st->r_theta) return CROWDSIM_EINVAL;
     if (B == 0) return CROWDSIM_OK;
@@ -274,13 +280,16 @@ extern "C" int crowdsim_lookahead_pack(const crowdsim_params *prm, int B, int N,
     const int threads = G.EPB * G.L;
     const int blocks = (B + G.EPB - 1) / G.EPB;
     size_t smem = cs::stage_bytes(G.EPB, G.L, G.k.nb_alloc, threads);
-    smem += (size_t)G.EPB * 48 + (size_t)A * 16 + (size_t)G.EPB * G.L * 8 + (size_t)A * N * 13 * sizeof(float);
+    const bool hlin = prm->human_policy == CROWDSIM_HUMANS_LINEAR;
+    smem += (size_t)G.EPB * 48 + (size_t)A * 16 + (size_t)G.EPB * G.L * (hlin ? 16 : 8) + (size_t)A * N * 13 * sizeof(float);
     if (smem > 227 * 1024) return CROWDSIM_EUNSUPPORTED;
     if (smem > 48 * 1024) {
-        cudaError_t err = cudaFuncSetAttribute(cs::lookahead_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t err = hlin ? cudaFuncSetAttribute(cs::lookahead_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                               : cudaFuncSetAttribute(cs::lookahead_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (err != cudaSuccess) return (int)err;
     }
-    cs::lookahead_kernel<<<blocks, threads, smem, (cudaStream_t)stream>>>(G);
+    if (hlin) cs::lookahead_kernel<true><<<blocks, threads, smem, (cudaStream_t)stream>>>(G);
+    else cs::lookahead_kernel<false><<<blocks, threads, smem, (cudaStream_t)stream>>>(G);
     ++cs::g_launches;
     return (int)cudaGetLastError();
 }
@@ -289,7 +298,7 @@ extern "C" int crowdsim_lookahead_humans(const crowdsim_params *prm, int B, int 
                                          double *next_h_pos, double *next_h_vel, void *stream)
 {
     if (!prm || !st || !next_h_pos || !next_h_vel || B < 0 || N < 1) return CROWDSIM_EINVAL;
-    if (N > CROWDSIM_MAX_HUMANS || prm->max_neighbors > CROWDSIM_MAX_NEIGHBORS) return CROWDSIM_EUNSUPPORTED;
+    if (N > CROWDSIM_MAX_HUMANS || prm->max_neighbors > CROWDSIM_MAX_NEIGHBORS || !cs::policies_supported(prm)) return CROWDSIM_EUNSUPPORTED;
     if (!st->h_pos || !st->h_vel || !st->h_goal || !st->h_attr || !st->r_pos || !st->r_vel || !st->r_attr) return CROWDSIM_EINVAL;
     if (B == 0) return CROWDSIM_OK;
     cs::NextArgs G;
@@ -299,11 +308,14 @@ extern "C" int crowdsim_lookahead_humans(const crowdsim_params *prm, int B, int 
     const int blocks = (B + G.EPB - 1) / G.EPB;
     const size_t smem = cs::stage_bytes(G.EPB, G.L, G.k.nb_alloc, threads);
     if (smem > 227 * 1024) return CROWDSIM_EUNSUPPORTED;
+    const bool hlin = prm->human_policy == CROWDSIM_HUMANS_LINEAR;
     if (smem > 48 * 1024) {
-        cudaError_t err = cudaFuncSetAttribute(cs::lookahead_humans_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t err = hlin ? cudaFuncSetAttribute(cs::lookahead_humans_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                               : cudaFuncSetAttribute(cs::lookahead_humans_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (err != cudaSuccess) return (int)err;
     }
-    cs::lookahead_humans_kernel<<<blocks, threads, smem, (cudaStream_t)stream>>>(G);
+    if (hlin) cs::lookahead_humans_kernel<true><<<blocks, threads, smem, (cudaStream_t)stream>>>(G);
+    else cs::lookahead_humans_kernel<false><<<blocks, threads, smem, (cudaStream_t)stream>>>(G);
     ++cs::g_launches;
     return (int)cudaGetLastError();
 }

@@ -51,6 +51,8 @@ namespace cs {
 // interleave (profiles/r02_multi_straight_lines.txt: launch 72.9 -> 71.5 us); 0 = the branchy form of the single-step kernel.
 // ROT: the robot is a unicycle (CROWDSIM_ROBOT_EXTERNAL_ROT, agent.py:115-135). A template parameter so that the double
 // precision cos / sin / fmod code (12 % of the round-1 kernel's SASS) is only present in the kernels that execute it.
+// LIN (kLinHumans | kLinRobot, crowdsim_common.cuh): humans and / or the robot follow Linear.predict (linear.py:15-22) instead
+// of ORCA; selected at compile time like ROT, so the ORCA instantiations (LIN = 0) are the same code as without it.
 #ifndef CS_FLAT_WPB
 #define CS_FLAT_WPB 4
 #endif
@@ -64,13 +66,15 @@ namespace cs {
 #define CS_FLAT_MINBLOCKS_MULTI 4
 #endif
 
-template <int N, int STAGE = 99, bool ROT = false, bool MULTI = false, bool WARPQ = MULTI>
+template <int N, int STAGE = 99, bool ROT = false, bool MULTI = false, bool WARPQ = MULTI, int LIN = 0>
 __global__ void __launch_bounds__(32 * CS_FLAT_WPB, (MULTI ? CS_FLAT_MINBLOCKS_MULTI : CS_FLAT_MINBLOCKS) * 4 / CS_FLAT_WPB)
 step_flat_kernel(const __grid_constant__ StepArgs A)
 {
     static_assert(STAGE == 99 || !MULTI, "stage cut-offs exist for the single-step kernel only");
     static_assert(!(ROT && MULTI), "a unicycle robot needs an external action every step");
     static_assert(WARPQ || !MULTI, "the multi-step kernel has no block barrier: warps run ahead of each other");
+    static_assert(!(ROT && (LIN & kLinRobot)), "a linear robot is holonomic");
+    constexpr bool HLIN = (LIN & kLinHumans) != 0, RLIN = (LIN & kLinRobot) != 0;
     if constexpr (STAGE == 0) return;
     using namespace orca;
     constexpr int L = N + 1, M = N, EPW = 32 / L, WPB = CS_FLAT_WPB;
@@ -109,7 +113,7 @@ step_flat_kernel(const __grid_constant__ StepArgs A)
             pos = ld2(A.st.r_pos, e); vel = ld2(A.st.r_vel, e); goal = ld2(A.st.r_goal, e); attr = ld2(A.st.r_attr, e);
             gtime = A.st.g_time[e];
             if (ROT) theta = A.st.r_theta[e];
-            if (k.robot_policy != CROWDSIM_ROBOT_ORCA) ext = ld2(A.io.action, e);
+            if (!RLIN && k.robot_policy != CROWDSIM_ROBOT_ORCA) ext = ld2(A.io.action, e);
             if (A.has_ep) { ep_t = A.ep.ep_steps[e]; ep_ret = A.ep.ep_return[e]; ep_tc = A.ep.ep_too_close[e]; ep_mds = A.ep.ep_min_dist_sum[e]; ep_c = A.ep.ep_case[e]; }
             if (A.has_ar) { if (!MULTI) slot_state = ld_relaxed_u8(A.ar.n_state + e); want_flag = A.ar.want[e]; }
         }
@@ -138,7 +142,9 @@ step_flat_kernel(const __grid_constant__ StepArgs A)
     const float fpx = (float)pos.x, fpy = (float)pos.y, fvx = (float)vel.x, fvy = (float)vel.y;
     const float frh = (float)(attr.x + 0.01 + k.human_safety_space);     // my radius as seen by a human observer
     const float frr = (float)(attr.x + 0.01 + k.robot_safety_space);     // ... by the robot
-    const bool solves = live && (!is_robot || k.robot_policy == CROWDSIM_ROBOT_ORCA);
+    // (linear humans do not solve; with a linear robot too nobody does, and the solver below folds away)
+    const bool solves = (LIN == (kLinHumans | kLinRobot)) ? false
+                      : live && (!is_robot || k.robot_policy == CROWDSIM_ROBOT_ORCA) && !(HLIN && !is_robot);
 
     // ---- orca.py:113-115 preferred velocity (float64) ----
     const double gvx = goal.x - pos.x, gvy = goal.y - pos.y;
@@ -353,7 +359,8 @@ step_flat_kernel(const __grid_constant__ StepArgs A)
     // ---- robot velocity of this step, broadcast inside the env ----
     double ax = 0, ay = 0, rvx = 0, rvy = 0;
     if (is_robot) {
-        if (k.robot_policy == CROWDSIM_ROBOT_ORCA) { ax = (double)nv.x; ay = (double)nv.y; rvx = ax; rvy = ay; }
+        if constexpr (RLIN) { const double2 lv = linear_velocity(pos, goal, attr.y); ax = lv.x; ay = lv.y; rvx = ax; rvy = ay; }
+        else if (k.robot_policy == CROWDSIM_ROBOT_ORCA) { ax = (double)nv.x; ay = (double)nv.y; rvx = ax; rvy = ay; }
         else if (ROT) { ax = ext.x; ay = ext.y; rvx = ax * cos(ay + theta); rvy = ax * sin(ay + theta); }      // crowd_sim.py:340-341
         else { ax = ext.x; ay = ext.y; rvx = ax; rvy = ay; }
     }
@@ -469,13 +476,14 @@ step_flat_kernel(const __grid_constant__ StepArgs A)
         act_flag = (uint8_t)__shfl_sync(CS_FULL, (int)act_flag, rl);
     }
     if (live && !is_robot && !install) {
-        // agent.py:122-135 holonomic step with the ORCA action (float32 values widened)
-        const double hx = (double)nv.x, hy = (double)nv.y;
+        // agent.py:122-135 holonomic step with the ORCA action (float32 values widened) or the Linear action (float64)
+        double hx = (double)nv.x, hy = (double)nv.y;
+        if constexpr (HLIN) { const double2 lv = linear_human_velocity(pos, goal, attr.y); hx = lv.x; hy = lv.y; }
         pos = make_double2(pos.x + hx * dt, pos.y + hy * dt); vel = make_double2(hx, hy);
         if constexpr (MULTI) dirty_kin = true;
         else {
             st2(A.st.h_pos, hi, pos); st2(A.st.h_vel, hi, vel);
-            if (A.io.obs32) reinterpret_cast<float4 *>(A.io.obs32)[hi] = make_float4((float)pos.x, (float)pos.y, nv.x, nv.y);
+            if (A.io.obs32) reinterpret_cast<float4 *>(A.io.obs32)[hi] = make_float4((float)pos.x, (float)pos.y, HLIN ? (float)hx : nv.x, HLIN ? (float)hy : nv.y);
         }
     }
     }   // step loop

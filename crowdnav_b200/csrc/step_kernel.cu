@@ -86,9 +86,11 @@ namespace cs {
 // MID = false: the generic kernel of round 1 (RVO2's sequential code on per-thread shared-memory columns; any
 // max_neighbors <= 10; kept as the A/B partner of the two fast kernels in the tests: crowdsim_debug_force_generic).
 // MID = true: the crowd kernel for N > 5 (step_mid.cuh: register-resident lines, speculative LPs, compacted lp3).
-template <bool MID>
+// LIN: linear humans / robot (crowdsim_common.cuh: kLinHumans, kLinRobot), a compile-time choice as in step_flat_kernel.
+template <bool MID, int LIN = 0>
 __global__ void __launch_bounds__(MID ? 128 : 256, MID ? CS_MID_MINBLOCKS : 1) step_kernel(const __grid_constant__ StepArgs A)
 {
+    constexpr bool HLIN = (LIN & kLinHumans) != 0, RLIN = (LIN & kLinRobot) != 0;
     extern __shared__ __align__(16) unsigned char smem[];
     __shared__ int s_qcount;
     const int T = blockDim.x, tid = threadIdx.x;
@@ -121,8 +123,9 @@ __global__ void __launch_bounds__(MID ? 128 : 256, MID ? CS_MID_MINBLOCKS : 1) s
 
     // ---- ORCA solves: every human lane; the robot lane iff the robot runs ORCA ----
     orca::V2 nv = orca::mk(0.f, 0.f);
-    const bool solve = live && (!is_robot || k.robot_policy == CROWDSIM_ROBOT_ORCA) && !(A.act_only && !is_robot);
-    if constexpr (MID) nv = mid_solve<kMidM>(s, k, solve, le, a, N, L, pos, goal, attr.y, tid, T, s.lines, &s_qcount);
+    const bool solve = live && (!is_robot || k.robot_policy == CROWDSIM_ROBOT_ORCA) && !(A.act_only && !is_robot) && !(HLIN && !is_robot);
+    if constexpr (LIN == (kLinHumans | kLinRobot)) (void)solve;      // nobody runs ORCA
+    else if constexpr (MID) nv = mid_solve<kMidM>(s, k, solve, le, a, N, L, pos, goal, attr.y, tid, T, s.lines, &s_qcount);
     else if (solve) nv = orca_predict(s, k, le, a, N, L, pos, goal, attr.y, tid, T);
 
     if (A.act_only) {
@@ -134,7 +137,8 @@ __global__ void __launch_bounds__(MID ? 128 : 256, MID ? CS_MID_MINBLOCKS : 1) s
     double ax = 0, ay = 0;            // raw action: (vx, vy) or (v, r)
     double2 rvel = make_double2(0, 0); // world-frame velocity used by the collision test
     if (live && is_robot) {
-        if (k.robot_policy == CROWDSIM_ROBOT_ORCA) { ax = (double)nv.x; ay = (double)nv.y; rvel = make_double2(ax, ay); }
+        if constexpr (RLIN) { rvel = linear_velocity(pos, goal, attr.y); ax = rvel.x; ay = rvel.y; }
+        else if (k.robot_policy == CROWDSIM_ROBOT_ORCA) { ax = (double)nv.x; ay = (double)nv.y; rvel = make_double2(ax, ay); }
         else {
             const double2 act = ld2(A.io.action, e); ax = act.x; ay = act.y;
             if (k.robot_policy == CROWDSIM_ROBOT_EXTERNAL_ROT) rvel = make_double2(ax * cos(ay + theta), ax * sin(ay + theta));  // crowd_sim.py:340-341
@@ -230,14 +234,15 @@ __global__ void __launch_bounds__(MID ? 128 : 256, MID ? CS_MID_MINBLOCKS : 1) s
         if (install && is_robot) st_release_u8(A.ar.n_state + e, CROWDSIM_SLOT_EMPTY);
     }
     if (live && !is_robot && !install) {
-        // agent.py:122-135 holonomic step with the ORCA action (float32 values widened)
-        const double hx = (double)nv.x, hy = (double)nv.y;
+        // agent.py:122-135 holonomic step with the ORCA action (float32 values widened) or the Linear action (float64)
+        double hx = (double)nv.x, hy = (double)nv.y;
+        if constexpr (HLIN) { const double2 lv = linear_human_velocity(pos, goal, attr.y); hx = lv.x; hy = lv.y; }
         const size_t i = (size_t)e * N + a;
         const double2 np_ = make_double2(pos.x + hx * dt, pos.y + hy * dt);
         if (A.lookahead) { st2(A.la_pos, i, np_); st2(A.la_vel, i, make_double2(hx, hy)); return; }   // agent.py:63-74, nothing mutated
         st2(A.st.h_pos, i, np_);
         st2(A.st.h_vel, i, make_double2(hx, hy));
-        if (A.io.obs32) reinterpret_cast<float4 *>(A.io.obs32)[i] = make_float4((float)np_.x, (float)np_.y, nv.x, nv.y);
+        if (A.io.obs32) reinterpret_cast<float4 *>(A.io.obs32)[i] = make_float4((float)np_.x, (float)np_.y, HLIN ? (float)hx : nv.x, HLIN ? (float)hy : nv.y);
     }
 }
 
@@ -307,19 +312,36 @@ static int sm_count()
     return cache[dev];
 }
 
+// n_steps launches of the crowd kernel (mid) or of the generic kernel for one policy combination
+template <int LIN>
+static int launch_crowd(const StepArgs &A, bool mid, int blocks, int threads, size_t smem, int n_steps, cudaStream_t stream)
+{
+    if (smem > 48 * 1024) {                                  // (a per-device attribute; setting it again is cheap)
+        cudaError_t err = mid ? cudaFuncSetAttribute(step_kernel<true, LIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                              : cudaFuncSetAttribute(step_kernel<false, LIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (err != cudaSuccess) return (int)err;
+    }
+    for (int rep = 0; rep < n_steps; ++rep) {
+        if (mid) step_kernel<true, LIN><<<blocks, threads, smem, stream>>>(A);
+        else step_kernel<false, LIN><<<blocks, threads, smem, stream>>>(A);
+        ++g_launches;
+    }
+    return (int)cudaGetLastError();
+}
+
 static int launch(const crowdsim_params *prm, int B, int N, const crowdsim_state *st, const crowdsim_step_io *io,
                   const crowdsim_episodes *ep, const crowdsim_autoreset *ar, int act_only, int n_steps, cudaStream_t stream,
                   double *la_pos = nullptr, double *la_vel = nullptr)
 {
     if (!prm || !st || !io || B < 0 || N < 0 || n_steps < 1) return CROWDSIM_EINVAL;
-    if (N > CROWDSIM_MAX_HUMANS || prm->max_neighbors > CROWDSIM_MAX_NEIGHBORS) return CROWDSIM_EUNSUPPORTED;
+    if (N > CROWDSIM_MAX_HUMANS || prm->max_neighbors > CROWDSIM_MAX_NEIGHBORS || !policies_supported(prm)) return CROWDSIM_EUNSUPPORTED;
     if (N > 0 && (!st->h_pos || !st->h_vel || !st->h_goal || !st->h_attr)) return CROWDSIM_EINVAL;
     if (!st->r_pos || !st->r_vel || !st->r_goal || !st->r_attr || !st->g_time) return CROWDSIM_EINVAL;
     if (prm->robot_policy == CROWDSIM_ROBOT_EXTERNAL_ROT && !st->r_theta) return CROWDSIM_EINVAL;
     if (act_only) { if (!io->action_out) return CROWDSIM_EINVAL; }
     else {
         if (!io->reward || !io->dmin || !io->done || !io->info) return CROWDSIM_EINVAL;
-        if (prm->robot_policy != CROWDSIM_ROBOT_ORCA && !io->action) return CROWDSIM_EINVAL;
+        if (prm->robot_policy != CROWDSIM_ROBOT_ORCA && prm->robot_policy != CROWDSIM_ROBOT_LINEAR && !io->action) return CROWDSIM_EINVAL;
     }
     if (ep && !act_only && (!ep->ep_case || !ep->ep_steps || !ep->ep_return || !ep->ep_too_close || !ep->ep_min_dist_sum ||
                             !ep->discount || !ep->res_info || !ep->res_steps || !ep->res_time || !ep->res_return ||
@@ -337,6 +359,7 @@ static int launch(const crowdsim_params *prm, int B, int N, const crowdsim_state
     if (A.has_ep) A.ep = *ep; else memset(&A.ep, 0, sizeof(A.ep));
     A.has_ar = (ar != nullptr && !act_only);
     if (A.has_ar) A.ar = *ar; else memset(&A.ar, 0, sizeof(A.ar));
+    const int lin = act_only ? 0 : lin_bits(prm);    // (orca_act: the robot's ORCA decision only, whatever the humans run)
     if (act_only && N >= 1 && N <= 5 && !g_force_generic) {
         const int blocks = (B + 127) / 128;
         switch (N) {
@@ -355,27 +378,30 @@ static int launch(const crowdsim_params *prm, int B, int N, const crowdsim_state
         const int blocks = (B + epb - 1) / epb;
         const bool rot = A.k.robot_policy == CROWDSIM_ROBOT_EXTERNAL_ROT;
         // n steps in one launch with the state in registers: closed-loop only (the robot decides on device)
-        const bool multi = n_steps > 1 && A.k.robot_policy == CROWDSIM_ROBOT_ORCA;
+        const bool multi = n_steps > 1 && (A.k.robot_policy == CROWDSIM_ROBOT_ORCA || A.k.robot_policy == CROWDSIM_ROBOT_LINEAR);
         const int reps = multi ? 1 : n_steps;
         if (multi) A.n_steps = n_steps;
         // linearProgram3 queue of the single-step kernel: per warp when the launch leaves SMs mostly empty (latency-bound: no
         // block barrier, 2-4 % faster at 1 k - 4 k envs), per block when the chip is full (issue-bound: one warp runs the pass
         // for the whole block, 3-5 % faster at 64 k - 1 M envs). Measured with scripts/latency_probe.cu in round 1.
         const bool warpq = blocks * CS_FLAT_WPB <= 12 * sm_count();
-        #define CS_FLAT_LAUNCH(NN) do { if (multi) step_flat_kernel<NN, 99, false, true, true><<<blocks, 32 * CS_FLAT_WPB, 0, stream>>>(A); \
-                                        else if (rot) step_flat_kernel<NN, 99, true, false, true><<<blocks, 32 * CS_FLAT_WPB, 0, stream>>>(A); \
-                                        else if (warpq) step_flat_kernel<NN, 99, false, false, true><<<blocks, 32 * CS_FLAT_WPB, 0, stream>>>(A); \
-                                        else step_flat_kernel<NN, 99, false, false, false><<<blocks, 32 * CS_FLAT_WPB, 0, stream>>>(A); } while (0)
+        #define CS_FLAT_LAUNCH(NN, LN) do { if (multi) step_flat_kernel<NN, 99, false, true, true, LN><<<blocks, 32 * CS_FLAT_WPB, 0, stream>>>(A); \
+                                            else if (rot) step_flat_kernel<NN, 99, !((LN) & kLinRobot), false, true, LN><<<blocks, 32 * CS_FLAT_WPB, 0, stream>>>(A); /* (never with a linear robot) */ \
+                                            else if (warpq) step_flat_kernel<NN, 99, false, false, true, LN><<<blocks, 32 * CS_FLAT_WPB, 0, stream>>>(A); \
+                                            else step_flat_kernel<NN, 99, false, false, false, LN><<<blocks, 32 * CS_FLAT_WPB, 0, stream>>>(A); } while (0)
+        #define CS_FLAT_LAUNCH_N(NN) do { switch (lin) { case 0: CS_FLAT_LAUNCH(NN, 0); break; case 1: CS_FLAT_LAUNCH(NN, 1); break; \
+                                                         case 2: CS_FLAT_LAUNCH(NN, 2); break; default: CS_FLAT_LAUNCH(NN, 3); break; } } while (0)
         for (int rep = 0; rep < reps; ++rep) {
             switch (N) {
-                case 1: CS_FLAT_LAUNCH(1); break;
-                case 2: CS_FLAT_LAUNCH(2); break;
-                case 3: CS_FLAT_LAUNCH(3); break;
-                case 4: CS_FLAT_LAUNCH(4); break;
-                default: CS_FLAT_LAUNCH(5); break;
+                case 1: CS_FLAT_LAUNCH_N(1); break;
+                case 2: CS_FLAT_LAUNCH_N(2); break;
+                case 3: CS_FLAT_LAUNCH_N(3); break;
+                case 4: CS_FLAT_LAUNCH_N(4); break;
+                default: CS_FLAT_LAUNCH_N(5); break;
             }
             ++g_launches;
         }
+        #undef CS_FLAT_LAUNCH_N
         #undef CS_FLAT_LAUNCH
         return (int)cudaGetLastError();
     }
@@ -383,17 +409,12 @@ static int launch(const crowdsim_params *prm, int B, int N, const crowdsim_state
     const int blocks = (B + A.EPB - 1) / A.EPB;
     const bool mid = !g_force_generic && N > 5;              // (N = 0 and the forced A/B route stay on the generic kernel)
     const size_t smem = mid ? stage_bytes_mid(A.EPB, A.L, mid_lp3_floats()) : stage_bytes(A.EPB, A.L, A.k.nb_alloc, threads);
-    if (smem > 48 * 1024) {                                  // (a per-device attribute; setting it again is cheap)
-        cudaError_t err = mid ? cudaFuncSetAttribute(step_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                              : cudaFuncSetAttribute(step_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (err != cudaSuccess) return (int)err;
+    switch (lin) {
+        case 0: return launch_crowd<0>(A, mid, blocks, threads, smem, n_steps, stream);
+        case 1: return launch_crowd<1>(A, mid, blocks, threads, smem, n_steps, stream);
+        case 2: return launch_crowd<2>(A, mid, blocks, threads, smem, n_steps, stream);
+        default: return launch_crowd<3>(A, mid, blocks, threads, smem, n_steps, stream);
     }
-    for (int rep = 0; rep < n_steps; ++rep) {
-        if (mid) step_kernel<true><<<blocks, threads, smem, stream>>>(A);
-        else step_kernel<false><<<blocks, threads, smem, stream>>>(A);
-        ++g_launches;
-    }
-    return (int)cudaGetLastError();
 }
 
 }  // namespace cs

@@ -107,7 +107,7 @@ extern "C" int crowdsim_human_times(const crowdsim_params *prm, int B, int N, co
                                     double *g_time_out, double *final_pos, int max_steps, void *stream)
 {
     if (!prm || !st || !human_times || !g_time_out || B < 0 || N < 1 || max_steps < 0) return CROWDSIM_EINVAL;
-    if (N > CROWDSIM_MAX_HUMANS || prm->max_neighbors > CROWDSIM_MAX_NEIGHBORS) return CROWDSIM_EUNSUPPORTED;
+    if (N > CROWDSIM_MAX_HUMANS || prm->max_neighbors > CROWDSIM_MAX_NEIGHBORS || !cs::policies_supported(prm)) return CROWDSIM_EUNSUPPORTED;
     if (!st->h_pos || !st->h_vel || !st->h_goal || !st->h_attr || !st->r_pos || !st->r_vel || !st->r_goal || !st->r_attr || !st->g_time) return CROWDSIM_EINVAL;
     if (B == 0) return CROWDSIM_OK;
     cs::TimesArgs A;

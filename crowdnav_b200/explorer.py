@@ -9,6 +9,7 @@ reference does (explorer.py:74-90).
 
 Robot policies:
   'orca'            the robot's ORCA solve is fused into the step kernel (test.py --policy orca)
+  'linear'          the robot's Linear.predict is fused into the step kernel (test.py --policy linear)
   a policy object   anything with .act_batch(env) -> [B][2] float64 device tensor of ActionXY (policy.make_sarl() ...)
 With update_memory=True the rollout also fills a memory.DeviceReplayMemory like Explorer.update_memory does
 (explorer.py:92-125; imitation-learning returns or target-network bootstraps).
@@ -137,10 +138,8 @@ class BatchedExplorer(object):
         rule = env.test_sim if phase == 'test' else env.train_val_sim
         env.set_case_queue((first_case + start) % env.case_size[phase], n_local, phase)    # wraps inside the phase like crowd_sim.py:283
         env.enable_autoreset(rule)
-        if self.robot_policy == 'orca':
-            env.set_robot_policy('orca')
-        else:
-            env.set_robot_policy('external_xy')
+        on_device = self.robot_policy in ('orca', 'linear')
+        env.set_robot_policy(self.robot_policy if on_device else 'external_xy')
         env.reset_seeds(rule=rule, use_queue=True)
         recorder = None
         if update_memory:
@@ -149,9 +148,9 @@ class BatchedExplorer(object):
             recorder = TrajectoryRecorder(env, self.memory, self.gamma, imitation_learning, self.target_model, om=om)
         side = torch.cuda.Stream(device=env.device)
         main = torch.cuda.current_stream(env.device)
-        # an ORCA robot decides on device: the episode loop of explorer.py:41-43 closes inside the kernel, several steps per
-        # launch (crowdsim_step_n); a recorded rollout or a host-side policy needs every step
-        chunk = max(1, int(steps_per_launch)) if (self.robot_policy == 'orca' and recorder is None) else 1
+        # an ORCA / Linear robot decides on device: the episode loop of explorer.py:41-43 closes inside the kernel, several
+        # steps per launch (crowdsim_step_n); a recorded rollout or a host-side policy needs every step
+        chunk = max(1, int(steps_per_launch)) if (on_device and recorder is None) else 1
         if chunk > 1:
             prefetch_every, check_every = 1, max(1, check_every // chunk)
         from .batched import max_episode_steps
@@ -164,7 +163,7 @@ class BatchedExplorer(object):
                     env.prefetch()
             if recorder is not None:
                 recorder.before_step()
-            if self.robot_policy == 'orca':
+            if on_device:
                 env.step(n_steps=chunk)
             else:
                 env.step(self.robot_policy.act_batch(env))

@@ -10,8 +10,9 @@
  *
  * What each entry point replaces in the reference (paths relative to /root/reference):
  *   crowdsim_step            crowd_sim/envs/crowd_sim.py:317-420 (CrowdSim.step, update=True) including the
- *                            N x Human.act -> ORCA.predict -> rvo2 doStep (crowd_sim/envs/policy/orca.py:82-132),
- *                            optionally the robot's own ORCA.predict (crowd_nav/utils/explorer.py:42), the
+ *                            N x Human.act -> ORCA.predict -> rvo2 doStep (crowd_sim/envs/policy/orca.py:82-132) or
+ *                            Linear.predict (crowd_sim/envs/policy/linear.py:15-22, human_policy),
+ *                            optionally the robot's own ORCA.predict / Linear.predict (crowd_nav/utils/explorer.py:42), the
  *                            per-step part of Explorer.run_k_episodes (explorer.py:41-72)
  *   crowdsim_step_n          the inner loop of Explorer.run_k_episodes for a robot that decides on device
  *                            (crowd_nav/utils/explorer.py:41-43: robot.act -> env.step, n times), closed on the GPU
@@ -41,12 +42,12 @@
 extern "C" {
 #endif
 
-#define CROWDSIM_ABI_VERSION 4
+#define CROWDSIM_ABI_VERSION 5
 
 /* error codes */
 #define CROWDSIM_OK            0
 #define CROWDSIM_EINVAL       (-1)   /* NULL required pointer / B,N out of range */
-#define CROWDSIM_EUNSUPPORTED (-2)   /* N > CROWDSIM_MAX_HUMANS, max_neighbors > CROWDSIM_MAX_NEIGHBORS, ... */
+#define CROWDSIM_EUNSUPPORTED (-2)   /* N > CROWDSIM_MAX_HUMANS, max_neighbors > CROWDSIM_MAX_NEIGHBORS, unknown policy, ... */
 #define CROWDSIM_ENODEVICE    (-3)   /* no CUDA device / wrong architecture */
 
 #define CROWDSIM_MAX_HUMANS     63   /* N + 1 (robot) agents of one env are staged together in shared memory */
@@ -63,6 +64,14 @@ extern "C" {
 #define CROWDSIM_ROBOT_EXTERNAL_XY  0  /* holonomic ActionXY supplied by the caller (CADRL/LSTM-RL/SARL/Linear) */
 #define CROWDSIM_ROBOT_ORCA         1  /* robot runs ORCA inside the step kernel (test.py --policy orca) */
 #define CROWDSIM_ROBOT_EXTERNAL_ROT 2  /* unicycle ActionRot (v, r) supplied by the caller (agent.py:115-118,133-135) */
+#define CROWDSIM_ROBOT_LINEAR       3  /* robot runs Linear inside the step kernel (test.py --policy linear): Linear.predict
+                                          (crowd_sim/envs/policy/linear.py:15-22) of its pre-step state, io->action unused */
+
+/* human_policy: env.config [humans] policy, crowd_sim/envs/policy/policy_factory.py:9-12 (crowd_sim.py:317-326 human.act) */
+#define CROWDSIM_HUMANS_ORCA   0  /* ORCA.predict (orca.py:82-132) */
+#define CROWDSIM_HUMANS_LINEAR 1  /* Linear.predict (linear.py:15-22): theta = atan2(gy - py, gx - px) in float64, velocity
+                                     (cos theta * v_pref, sin theta * v_pref); no neighbour scan. A human standing on its goal
+                                     steps +x (atan2(0, 0) = 0) like the reference's; PARKED slots of `mixed` stay still. */
 
 /* scenario rules: crowd_sim.py:84-153 */
 #define CROWDSIM_RULE_CIRCLE 0
@@ -91,6 +100,7 @@ typedef struct crowdsim_params {
     double robot_safety_space;        /* 0 (train.py:121-127 sets 0.15 for IL with an invisible robot) */
     int32_t robot_visible;            /* env.config [robot] visible; crowd_sim.py:325-327 */
     int32_t robot_policy;             /* CROWDSIM_ROBOT_* */
+    int32_t human_policy;             /* CROWDSIM_HUMANS_* (appended last: zero-filled initialisers mean ORCA humans) */
 } crowdsim_params;
 
 /* Agent state. Mutable arrays are updated in place by crowdsim_step (agent.py:122-135). */
@@ -110,7 +120,7 @@ typedef struct crowdsim_state {
 
 /* Per-step inputs / outputs of crowdsim_step. */
 typedef struct crowdsim_step_io {
-    const double *action; /* [B][2] robot action (vx,vy) or (v,r); ignored (may be NULL) for CROWDSIM_ROBOT_ORCA */
+    const double *action; /* [B][2] robot action (vx,vy) or (v,r); ignored (may be NULL) for CROWDSIM_ROBOT_ORCA / _LINEAR */
     double *action_out;   /* [B][2] or NULL: the holonomic velocity actually applied to the robot */
     double *reward;       /* [B] */
     double *dmin;         /* [B] min robot-human clearance this step (inf if N == 0) */
@@ -233,8 +243,8 @@ int crowdsim_step(const crowdsim_params *prm, int B, int N, crowdsim_state *st, 
 
 /*
  * n_steps lockstep env-steps in one call: exactly n_steps x crowdsim_step(prm, B, N, st, io, ep, ar) -- same final state,
- * same episode rows, same slot hand-overs; `io` holds the outputs of each env's LAST live step. With an ORCA robot
- * (CROWDSIM_ROBOT_ORCA) nothing leaves the device between the steps of the reference's episode loop
+ * same episode rows, same slot hand-overs; `io` holds the outputs of each env's LAST live step. With a robot that decides on
+ * device (CROWDSIM_ROBOT_ORCA or CROWDSIM_ROBOT_LINEAR) nothing leaves the device between the steps of the reference's episode loop
  * (crowd_nav/utils/explorer.py:41-43), so for N <= 5 the whole call is ONE kernel launch that keeps every env's state in
  * registers across the steps (one load, n_steps solves, one store); an env whose episode ends installs its prefetched next
  * scene on the spot and goes on (a second termination inside the same call finds the slot EMPTY and parks until the next
