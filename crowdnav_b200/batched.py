@@ -437,6 +437,9 @@ class BatchedCrowdSim(object):
         gt = torch.empty((B,), dtype=torch.float64, device=self.device)
         fp = torch.empty((B, N + 1, 2), dtype=torch.float64, device=self.device)
         prm = self.params(); st = self.state.struct()
+        # the centralised simulation has its own constants (neighborDist, maxNeighbors, timeHorizon = 10, 10, 5;
+        # crowd_sim.py:220), whatever the env's ORCA agents use
+        prm.neighbor_dist, prm.max_neighbors, prm.time_horizon = 10.0, 10, 5.0
         with torch.cuda.device(self.device):
             rc = self.lib.crowdsim_human_times(C.byref(prm), B, N, C.byref(st), _ptr(ht), _ptr(gt), _ptr(fp), int(max_steps), self._stream())
         _abi.check(rc, 'crowdsim_human_times')

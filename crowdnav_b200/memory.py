@@ -65,11 +65,12 @@ class TrajectoryRecorder(object):
         self.states = torch.zeros((B, self.T, N, F), dtype=torch.float32, device=dev)
         self.rewards = torch.zeros((B, self.T), dtype=torch.float64, device=dev)
         self.returns = torch.zeros((B, self.T), dtype=torch.float64, device=dev)
-        expo = env.time_step * env.robot_v_pref
-        # W[t][i] = pow(gamma, (t - i) * time_step * v_pref) for i <= t, else 0   (explorer.py:104-105)
-        w = [[pow(gamma, (t - i) * expo) if i <= t else 0.0 for i in range(self.T)] for t in range(self.T)]
+        dt, v_pref = env.time_step, env.robot_v_pref
+        # W[t][i] = pow(gamma, max(t - i, 0) * time_step * v_pref) for i <= t, else 0   (explorer.py:104-105), evaluated
+        # left to right as the reference does: ((t - i) * dt) * v_pref rounds differently from (t - i) * (dt * v_pref)
+        w = [[pow(gamma, (t - i) * dt * v_pref) if i <= t else 0.0 for i in range(self.T)] for t in range(self.T)]
         self.W = torch.tensor(w, dtype=torch.float64, device=dev)
-        self.gamma_bar = pow(gamma, expo)
+        self.gamma_bar = pow(gamma, dt * v_pref)                         # explorer.py:112
         self._t = None
         self._live = None
 

@@ -105,11 +105,13 @@ def discount_table(gamma, time_step, v_pref, n=128):
 
 
 class HostEpisodes(object):
-    def __init__(self, B, k, gamma=0.9, time_step=0.25, v_pref=1.0):
+    def __init__(self, B, k, gamma=0.9, time_step=0.25, v_pref=1.0, max_steps=128):
+        """max_steps: length of the discount table, at least the longest episode (steps beyond it count as undiscounted
+        to zero, like the kernels do)."""
         self.ep_case = np.full(B, -1, dtype=np.int32); self.ep_steps = np.zeros(B, dtype=np.int32)
         self.ep_return = np.zeros(B); self.ep_too_close = np.zeros(B, dtype=np.int32)
         self.ep_min_dist_sum = np.zeros(B)
-        self.discount = discount_table(gamma, time_step, v_pref)
+        self.discount = discount_table(gamma, time_step, v_pref, max(128, max_steps))
         self.res_info = np.zeros(k, dtype=np.uint8); self.res_steps = np.zeros(k, dtype=np.int32)
         self.res_time = np.zeros(k); self.res_return = np.zeros(k)
         self.res_too_close = np.zeros(k, dtype=np.int32); self.res_min_dist_sum = np.zeros(k)
@@ -230,7 +232,7 @@ def get_stats():
 def run_episodes(prm, N, seeds, rule='circle_crossing', gamma=0.9, robot_v_pref=1.0, max_steps=200, **reset_kw):
     """Run one episode per seed to termination (lockstep, finished envs frozen); returns HostEpisodes + state."""
     B = len(seeds)
-    st = HostState(B, N); io = HostStepIO(B); ep = HostEpisodes(B, B, gamma, prm.time_step, robot_v_pref)
+    st = HostState(B, N); io = HostStepIO(B); ep = HostEpisodes(B, B, gamma, prm.time_step, robot_v_pref, max_steps)
     ep.ep_case[:] = np.arange(B)
     reset(st, seeds, rule, ep=ep, robot_v_pref=robot_v_pref, **reset_kw)
     for _ in range(max_steps):

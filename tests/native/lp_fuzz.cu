@@ -1,7 +1,8 @@
 // lp_fuzz.cu -- CPU fuzz test (test infrastructure): the CUDA solver's arithmetic compiled FOR THE HOST
 // (crowdnav_b200/csrc/orca_device.cuh, orca_spec.cuh are __host__ __device__) against the C oracle
 // (oracle/rvo2_f32.h) on millions of random ORCA problems, bit for bit:
-//   A  make_line / make_line_sel            vs  orc_make_line
+//   A  make_line / make_line_sel / make_line_far + make_line_overlap   vs  orc_make_line, time horizon and time step drawn
+//      per case from {5, 3, 2.5, 10} s and {0.25, 0.1, 0.2, 1/30} s
 //   B  sequential lp2 + lp3 (shared-memory-column code path of the generic kernel, n <= 10)   vs  orc_lp2 / orc_lp3
 //   C  speculative lp1_all + lp2_scan (register path of the small-crowd kernel, n <= 5)        vs  orc_lp2
 //   D  lp3 as independent per-line sub-problems + lp3_outer_scan (the lane-parallel pass)      vs  orc_lp3
@@ -141,7 +142,7 @@ int main(int argc, char **argv)
 {
     const long cases = argc > 1 ? atol(argv[1]) : 200000;
     rng_state = argc > 2 ? strtoull(argv[2], nullptr, 10) * 2654435761ull + 88172645463325252ull : 88172645463325252ull;
-    long cov[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    long cov[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
     using namespace orca;
     for (int i = 1, q = 0; i <= 9; ++i) for (int j = 0; j < i; ++j, ++q) { int a, b; lp3_pair_of(q, a, b); if (a != i || b != j) { printf("lp3_pair_of(%d)\n", q); return 1; } }
     for (long c = 0; c < cases; ++c) {
@@ -150,6 +151,13 @@ int main(int argc, char **argv)
         orc_line ol[16];
         const float radius = uni(0.5f, 1.5f);
         orc_v2 opt = orc_mk(uni(-1.2f, 1.2f), uni(-1.2f, 1.2f));
+        // time horizon and time step of the env's config (default 5 s / 0.25 s; 0.1, 0.2 and 1/30 are not powers of two),
+        // converted the way the kernels' launch set-up does (crowdsim_common.cuh): inverses of the float32 values
+        static const double horizons[4] = {5.0, 3.0, 2.5, 10.0}, steps[4] = {0.25, 0.1, 0.2, 1.0 / 30.0};
+        const int hsel = rnd() % 4, tsel = rnd() % 4;
+        const float th = (float)horizons[hsel], dt = (float)steps[tsel];
+        const float inv_th = 1.0f / th, inv_dt = 1.0f / dt;
+        cov[8] += (hsel != 0); cov[9] += (tsel != 0);
         if (kind <= 1 || kind == 3) {
             // lines from a random crowd around an agent at the origin (kind 1: tight -> overlaps, infeasible LPs)
             const float spread = (kind == 1) ? 1.0f : 4.0f;
@@ -157,15 +165,15 @@ int main(int argc, char **argv)
             for (int k = 0; k < n; ++k) {
                 const orc_v2 po = orc_mk(uni(-spread, spread), uni(-spread, spread)), vo = orc_mk(uni(-1, 1), uni(-1, 1));
                 const float r = uni(0.2f, 0.5f), ro = uni(0.2f, 0.5f);
-                ol[k] = orc_make_line(p, v, r, po, vo, ro, 1.0f / 5.0f, 0.25f);
+                ol[k] = orc_make_line(p, v, r, po, vo, ro, inv_th, dt);
                 // ---- A: line construction ----
                 V2 lp, ld, sp, sd;
-                make_line(mk(p.x, p.y), mk(v.x, v.y), r, mk(po.x, po.y), mk(vo.x, vo.y), ro, 1.0f / 5.0f, 1.0f / 0.25f, lp, ld);
-                make_line_sel(mk(p.x, p.y), mk(v.x, v.y), r, mk(po.x, po.y), mk(vo.x, vo.y), ro, 1.0f / 5.0f, 1.0f / 0.25f, sp, sd);
+                make_line(mk(p.x, p.y), mk(v.x, v.y), r, mk(po.x, po.y), mk(vo.x, vo.y), ro, inv_th, inv_dt, lp, ld);
+                make_line_sel(mk(p.x, p.y), mk(v.x, v.y), r, mk(po.x, po.y), mk(vo.x, vo.y), ro, inv_th, inv_dt, sp, sd);
                 {   // straight-line form + overlap repair (multi-step kernel)
                     V2 fp, fd; bool ov;
-                    make_line_far(mk(p.x, p.y), mk(v.x, v.y), r, mk(po.x, po.y), mk(vo.x, vo.y), ro, 1.0f / 5.0f, fp, fd, ov);
-                    if (ov) make_line_overlap(mk(p.x, p.y), mk(v.x, v.y), r, mk(po.x, po.y), mk(vo.x, vo.y), ro, 1.0f / 0.25f, fp, fd);
+                    make_line_far(mk(p.x, p.y), mk(v.x, v.y), r, mk(po.x, po.y), mk(vo.x, vo.y), ro, inv_th, fp, fd, ov);
+                    if (ov) make_line_overlap(mk(p.x, p.y), mk(v.x, v.y), r, mk(po.x, po.y), mk(vo.x, vo.y), ro, inv_dt, fp, fd);
                     if (!same(fp.x, lp.x) || !same(fp.y, lp.y) || !same(fd.x, ld.x) || !same(fd.y, ld.y)) { printf("A far/overlap line mismatch\n"); return 1; }
                 }
                 if (!same(lp.x, ol[k].point.x) || !same(lp.y, ol[k].point.y) || !same(ld.x, ol[k].dir.x) || !same(ld.y, ol[k].dir.y) ||
@@ -188,6 +196,6 @@ int main(int argc, char **argv)
         if (!check_sorted_insert(cov)) { printf("case %ld\n", c); return 1; }
         if (!(check_order<5>(cov) && check_order<4>(cov) && check_order<2>(cov) && check_order<1>(cov))) { printf("case %ld\n", c); return 1; }
     }
-    printf("ok cases=%ld lp3_needed=%ld speculative_checked=%ld overlapping_pairs=%ld forced_parallel_lines=%ld neighbour_orders=%ld neighbour_ties=%ld lane_lp3_checked=%ld sorted_lists=%ld\n", cases, cov[0], cov[1], cov[2], cov[3], cov[4], cov[5], cov[6], cov[7]);
+    printf("ok cases=%ld lp3_needed=%ld speculative_checked=%ld overlapping_pairs=%ld forced_parallel_lines=%ld neighbour_orders=%ld neighbour_ties=%ld lane_lp3_checked=%ld sorted_lists=%ld other_horizon=%ld other_time_step=%ld\n", cases, cov[0], cov[1], cov[2], cov[3], cov[4], cov[5], cov[6], cov[7], cov[8], cov[9]);
     return 0;
 }

@@ -1,6 +1,6 @@
 """CPU fuzz of the CUDA solver's arithmetic: orca_device.cuh / orca_spec.cuh are __host__ __device__, so the exact code the
 kernels run is compiled for the host (nvcc, --fmad=false, -ffp-contract=off) and compared bit for bit with the C oracle on
-millions of random ORCA problems -- line construction, sequential lp2/lp3, the speculative lp1_all + lp2_scan path and the
+millions of random ORCA problems -- line construction (at several time horizons and time steps), sequential lp2/lp3, the speculative lp1_all + lp2_scan path and the
 lane-parallel formulation of lp3 (independent per-line sub-problems + outer scan). See tests/native/lp_fuzz.cu."""
 import os
 import subprocess
@@ -32,3 +32,5 @@ def test_host_compiled_solver_matches_oracle_bitwise(fuzz_binary, seed):
     assert int(fields['sorted_lists']) == 1000000                                                    # part H
     assert int(fields['lane_lp3_checked']) == int(fields['lp3_needed'])                              # part F
     assert int(fields['neighbour_orders']) == 4000000 and int(fields['neighbour_ties']) > 1000000    # part E, M = 5, 4, 2, 1
+    # line construction away from the default 5 s horizon / 0.25 s step (3 of 4 cases each)
+    assert int(fields['other_horizon']) > 700000 and int(fields['other_time_step']) > 700000
